@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- Nexmark-shaped streaming HashJoin (headline) and HashAgg (secondary) throughput.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs value,e2e,agg,chain,cpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs value,e2e,agg,chain,cpu] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], "Nexmark q7/q8 streaming HashJoin (bid x auction) 1xB200, 10M build
 rows in HBM"; SURVEY 8(d) cfg3):  the auction side (10 000 000 rows: id, seller, category, expires)
@@ -25,6 +25,8 @@ RWGPU_EXCHANGE=nccl selects partition + NCCL all-to-all-v instead.
             committed ncu capture (profiles/r1_traffic.json).  `clocks`: in-process NVML samples during the region.
 `--impl reference`: the CPU restatement of the reference algorithm (oracle/fastcpu.cc, one
 single-threaded actor per host core, inputs pre-partitioned by vnode) on a bounded sample.
+`--dump-outputs DIR`: after the timed steps, the join output of the last one as DIR/<name>.npy (see dump_outputs), so
+that two builds can be compared output for output: the inputs are generated from fixed seeds.
 """
 import argparse
 import contextlib
@@ -42,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (which may be read-only)
 
 N_BUILD = 10_000_000
 BATCH = 1 << 20
@@ -308,6 +311,35 @@ def vnode_of_int64(keys):
 
 
 CHECKSUM_WEIGHTS = (3, 31, 5, 7, 11, 1, 17, 19)  # oracle/fastcpu.cc OutBuilder::append
+
+DUMP_COLUMNS = ("bid_auction", "bid_date_time", "bid_bidder", "bid_price", "auction_id", "auction_seller", "auction_category",
+                "auction_expires")
+DUMP_MAX_ROWS = 1 << 19  # 8 float64 columns + float32 ops: ~36 MB
+DUMP_SEED = 0x5EED
+
+
+def dump_outputs(out_dir, view):
+    """Writes the output view of a join push as out_dir/<name>.npy.  The visible rows are sorted by all columns (the row
+    order of a join's output is not part of its result) and a fixed, seeded sample of at most DUMP_MAX_ROWS of them is kept:
+    ops.npy (float32) and one float64 array per output column (exact: every value of the workload is below 2^53).
+    summary.npy covers ALL visible rows: [row count, low and high 32 bits of the order-independent checksum of
+    DeviceView.checksum(CHECKSUM_WEIGHTS)]."""
+    os.makedirs(out_dir, exist_ok=True)
+    ops = view.ops().cpu().numpy()
+    cols = [view.column(k).cpu().numpy() for k in range(view.n_cols)]
+    vis = view.visible()
+    if vis is not None:
+        keep = vis.cpu().numpy()
+        ops, cols = ops[keep], [c[keep] for c in cols]
+    order = np.lexsort([ops] + cols[::-1])  # primary key: column 0
+    n = len(ops)
+    if n > DUMP_MAX_ROWS:
+        order = order[np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_ROWS, replace=False))]
+    rows, cs = view.checksum(CHECKSUM_WEIGHTS)
+    np.save(os.path.join(out_dir, "summary.npy"), np.array([rows, cs & 0xFFFFFFFF, cs >> 32], np.float64))
+    np.save(os.path.join(out_dir, "ops.npy"), ops[order].astype(np.float32))
+    for name, c in zip(DUMP_COLUMNS, cols):
+        np.save(os.path.join(out_dir, name + ".npy"), c[order].astype(np.float64))
 
 
 def cpu_topology():
@@ -608,6 +640,7 @@ def run_ours(args):
                 return out
 
             tl = []  # BENCH_TRACE: host timeline (never for a reported number)
+            last_out = [None]  # output view of the last step run (valid until the next push reuses its output set)
 
             def run_steps(lo, hi, each=None):
                 """steps lo..hi-1, push s+1 launched before push s is collected (two output sets)"""
@@ -625,6 +658,7 @@ def run_ours(args):
                         tl.append((s, 1e3 * (t_b - t_a), 1e3 * (time.perf_counter() - t_b)))
                 o = collect(hi - 1)
                 tot += o.n_rows
+                last_out[0] = o
                 if each:
                     each(o)
                 return tot
@@ -652,6 +686,8 @@ def run_ours(args):
             clocks = sampler.stop() if rank == 0 else None
             kern_ms, kern_n = device.profile(join, "join", False)
             launches = device.launches(join, "join") - l0
+            if args.dump_outputs and rank == 0:  # (before the verification pushes reuse the output sets)
+                dump_outputs(args.dump_outputs, last_out[0])
             if world > 1:
                 t = torch.tensor([ms], device="cuda", dtype=torch.float64)
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1261,7 +1297,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--legs", default="value,retract,hot,e2e,agg,q1,chain,generic,cpu",
                     help="comma list of: value,retract,hot,e2e,agg,q1,chain,generic,cpu (subset for ncu runs; retract needs value)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the join output of the last timed step of the value leg (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or "value" not in args.legs.split(",")):
+        ap.error("--dump-outputs needs --impl ours and the value leg")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     # stdout carries exactly ONE line (the JSON): everything a library prints there on its own (NCCL's "NCCL version ..."
     # banner at communicator creation, for one) is sent to stderr for the duration of the run

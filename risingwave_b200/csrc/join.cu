@@ -2378,13 +2378,22 @@ static int uni_finish(rwgpu_join* h, const JoinPending& pd, int64_t* out_rows, u
     hs.pad = hs.pad || first_match;
     hs.n_del = first_del;  // (the redo is probe-only: it counts no deletes)
   }
-  // bookkeeping: what the device really used, plus the upper bounds of the pushes enqueued after this one
+  // bookkeeping: what the device really used, plus the upper bounds of the pushes enqueued after this one.  Those pushes
+  // (still in h->pending: the caller has taken this one out) recorded the uncorrected bounds as their bases; their bases
+  // move by the same amount, so that their own collect removes exactly their share (with a stale base the bounds can
+  // wrap below zero, and the bucket-array growth loop never terminates)
   for (int s = 0; s < 2; s++) h->uni_dead[s] = hs.n_dead[s];
   {
     JoinSideHost& own = h->side[pd.S];
     const uint64_t n = (uint64_t)pd.ch.n, slack = (uint64_t)pd.grid * 8 * pd.pool_chunk;
-    own.n_rows = hs.log_next[pd.S] + (own.n_rows - (pd.ids_before + n + slack));
-    h->uni_keys = hs.n_keys[0] + (h->uni_keys - (pd.keys_before + n));
+    const uint64_t rows = hs.log_next[pd.S] + (own.n_rows - (pd.ids_before + n + slack));
+    const uint64_t keys = hs.n_keys[0] + (h->uni_keys - (pd.keys_before + n));
+    for (int i = 0; i < h->n_pending; i++) {
+      if (h->pending[i].S == pd.S) h->pending[i].ids_before += rows - own.n_rows;
+      h->pending[i].keys_before += keys - h->uni_keys;
+    }
+    own.n_rows = rows;
+    h->uni_keys = keys;
     h->uni_keys_exact = hs.n_keys[0];
   }
   hs.err = err;
